@@ -68,7 +68,12 @@ def parse():
                     help="N>1 only. sharded: the reference's Gaussian-sharded scheme (gsplat_distributed_renderer.py): scene split by "
                          "index across ranks, one camera per rank, all-to-all of the visible projected splats, gsplat semantics. "
                          "replicas: every rank holds the whole scene (configs/ddp.yaml style), no data-path collective.")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (rank 0) as DIR/<name>.npy, float32: "
+                         "the image, and radii / view-space gradient / raw-parameter gradients of a fixed seeded sample of Gaussians")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.config is None:
         args.config = 1 if world == 1 else 3
@@ -342,14 +347,17 @@ class Workload:
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(self, k, e2e):
+    def timed(self, k, e2e, keep_last=False):
         self.barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         if e2e:
             self.prefetch(0)
         for i in range(k):
-            self.step(i, e2e, i + 1 < k)
+            out = self.step(i, e2e, i + 1 < k)
+            if keep_last and i + 1 == k:
+                self.last_out = out
+            del out
             if not e2e:
                 self.step_done[i & 1].record()
             if i > 0:   # the host stays at most one step ahead in both loops, like a training loop that logs its loss
@@ -371,15 +379,19 @@ class Workload:
             ms = float(t[0])
         return ms
 
-    def run(self, steps, warmup, e2e=True, stages=True):
-        """-> dict(ms_total, ms_e2e, launches, stage_ms).  W untimed warm-up steps, then EXACTLY `steps` timed steps."""
+    def run(self, steps, warmup, e2e=True, stages=True, keep_outputs=False):
+        """-> dict(ms_total, ms_e2e, launches, stage_ms).  W untimed warm-up steps, then EXACTLY `steps` timed steps.
+        keep_outputs: self.outputs = host copies of what the last timed step computed (see host_outputs)."""
         from b200gs import ops
         for i in range(max(warmup, 3)):
             self.step(i)
         self.timed(min(steps, 16), False)      # untimed: lets the caching allocator settle into the timed loop's pattern
         l0 = _launch_count()
-        ms_total = self.timed(steps, False)
+        ms_total = self.timed(steps, False, keep_last=keep_outputs)
         l1 = _launch_count()
+        if keep_outputs:     # before the steps below overwrite the gradients
+            self.outputs = self.host_outputs(self.last_out)
+            del self.last_out
         ms_e2e = self.timed(steps, True) if e2e else None
         stage_ms = {}
         if stages:    # per-stage timing (CUDA events on the launching stream) for the roofline numbers
@@ -390,6 +402,25 @@ class Workload:
             stage_ms, _ = timer.summary_ms()
             ops.set_stage_timer(None)
         return {"ms_total": ms_total, "ms_e2e": ms_e2e, "launches": (l1 - l0) if l0 is not None else None, "stage_ms": stage_ms}
+
+    DUMP_ROWS = 1 << 16            # Gaussians sampled for the per-Gaussian arrays (16.5 MB at SH degree 3)
+    DUMP_IMAGE_BYTES = 32 << 20    # a larger image is sampled at a fixed seeded set of pixels
+
+    def host_outputs(self, out):
+        """Float32 host copies of what the caller of one step receives: the rendered image [3,H,W], and for a fixed seeded sample of
+        this rank's Gaussians (sorted indices) the radii, the view-space gradient and the gradients of the raw parameter tensors."""
+        n = self.model.gaussians["means"].shape[0]
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:self.DUMP_ROWS].sort().values.to(self.dev)
+        img = out["render"].detach()
+        if img.numel() * 4 > self.DUMP_IMAGE_BYTES:
+            pix = torch.randperm(img[0].numel(), generator=torch.Generator().manual_seed(1))[:self.DUMP_IMAGE_BYTES // 12]
+            img = img.reshape(img.shape[0], -1)[:, pix.sort().values.to(self.dev)]
+        res = {"render": img, "radii": out["radii"][rows]}
+        if out["viewspace_points"].grad is not None:
+            res["viewspace_points_grad"] = out["viewspace_points"].grad[rows]
+        for k, p in self.model.gaussians.items():
+            res[f"grad_{k}"] = p.grad[rows]
+        return {k: v.float().cpu().numpy() for k, v in res.items()}
 
     def views_per_s(self, ms, steps):
         return steps * self.world / (ms * 1e-3)
@@ -501,8 +532,14 @@ def main():
     if rank == 0:
         sampler.start()
     wl = Workload(N, W, H, args.mode, rank, world, local, sharded)
-    res = wl.run(args.steps, args.warmup)
+    dump = args.dump_outputs is not None and rank == 0
+    res = wl.run(args.steps, args.warmup, keep_outputs=dump)
     clocks = sampler.stop() if rank == 0 else None
+    if dump:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in wl.outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     ms_total, ms_e2e, stage_ms = res["ms_total"], res["ms_e2e"], res["stage_ms"]
     cot_bytes = int(wl.cot_host.numel() * 4)
     del wl

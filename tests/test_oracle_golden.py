@@ -115,29 +115,14 @@ def test_camera_restatement_matches_product_camera():
 
 
 def test_product_camera_matches_reference_cameras_class():
-    """b200gs.cameras.make_camera against the reference's own Cameras dataclass (baseline/_ref), when it is installed."""
-    import importlib.util
-    import os
-    import math
-    from conftest import ROOT
-    path = os.path.join(ROOT, "baseline", "_ref", "internal", "cameras", "cameras.py")
-    if not os.path.exists(path):
-        pytest.skip("baseline/_ref not present")
-    spec = importlib.util.spec_from_file_location("ref_cameras", path)
-    m = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(m)
-    from b200gs.scene import make_ring_cameras, ring_pose
-    W, H = 1920, 1080
-    fx = 0.5 * W / math.tan(math.radians(39.6) * 0.5)
-    for k in (0, 5, 17):
-        R, T = ring_pose(k)
-        cams = m.Cameras(R=R[None], T=T[None], fx=torch.tensor([fx]), fy=torch.tensor([fx]), cx=torch.tensor([W / 2.0]),
-                         cy=torch.tensor([H / 2.0]), width=torch.tensor([W], dtype=torch.int32),
-                         height=torch.tensor([H], dtype=torch.int32), appearance_id=torch.zeros(1, dtype=torch.int32),
-                         normalized_appearance_id=torch.zeros(1), distortion_params=None, camera_type=torch.zeros(1, dtype=torch.int32))
-        ref, mine = cams[0], make_ring_cameras(W, H)[k]
+    """b200gs.cameras.make_camera against what the reference's own Cameras dataclass derives for the same poses
+    (tests/golden/make_golden_cameras.py)."""
+    from b200gs.scene import make_ring_cameras
+    d = np.load(os.path.join(GOLDEN, "cameras_1920x1080.npz"))
+    cams = make_ring_cameras(1920, 1080)
+    for k in d["poses"].tolist():
         for name in ("world_to_camera", "full_projection", "camera_center", "fov_x", "fov_y"):
-            assert torch.equal(getattr(ref, name), getattr(mine, name)), name
+            assert torch.equal(torch.from_numpy(d[f"{name}_{k}"]), getattr(cams[k], name)), (name, k)
 
 
 def test_sh_degree4_matches_reference():
