@@ -41,7 +41,6 @@ _SIGNATURES = {
     "b200gs_project_fwd": (c_int32, [POINTER(B200gsView), c_int64] + [_P] * 4 + [_P] * 9 + [_P]),
     "b200gs_project_bwd": (c_int32, [POINTER(B200gsView), c_int64] + [_P] * 4 + [_P] * 2 + [_P] * 5 + [_P] * 4 + [_P]),
     "b200gs_project_fwd_raw": (c_int32, [POINTER(B200gsView), c_int64] + [_P] * 6 + [c_int32] + [_P] * 9 + [_P]),
-    "b200gs_project_bwd_raw": (c_int32, [POINTER(B200gsView), c_int64] + [_P] * 6 + [c_int32] + [_P] * 2 + [_P] * 5 + [_P] * 6 + [_P]),
     "b200gs_selective_adam": (c_int32, [c_int64, c_int32, _P, _P, _P, _P, _P, c_float, c_float, c_float, c_float, _P]),
     "b200gs_densify_stats": (c_int32, [c_int64, _P, _P, _P, c_int32, c_float, c_float, _P, _P, _P, _P]),
     "b200gs_knn_workspace_bytes": (c_size_t, [c_int64]),
@@ -60,18 +59,15 @@ _SIGNATURES = {
     "b200gs_blend_fwd_hits": (c_int32, [c_int32] * 4 + [_P] * 7 + [_P, c_int64, c_int64, _P, _P, _P, _P, _P]),
     "b200gs_blend_bwd": (c_int32, [c_int32] * 4 + [_P] * 7 + [_P, _P, _P, c_int64, c_int64, _P, c_float, c_float]
                          + [_P] * 5 + [_P]),
-    "b200gs_blend_bwd_to_rows": (c_int32, [c_int32] * 3 + [_P] * 7 + [_P, _P, _P, c_int64, c_int64, _P, c_float, c_float, _P, _P, _P]),
     "b200gs_project_bwd_rows": (c_int32, [POINTER(B200gsView), c_int64] + [_P] * 6 + [c_int32] + [_P] * 4 + [c_int32] + [_P] * 6 + [_P, c_int32] + [_P]),
     "b200gs_project_fwd_raw_multi": (c_int32, [POINTER(B200gsView), c_int32, c_int64] + [_P] * 6 + [c_int32] + [_P] * 7 + [_P]),
     "b200gs_project_bwd_rows_multi": (c_int32, [POINTER(B200gsView), c_int32, c_int64] + [_P] * 6 + [c_int32] + [_P] * 3 + [POINTER(c_void_p)] + [_P] * 6 + [_P]),
-    "b200gs_pack_rows_peer": (c_int32, [c_int64, c_int64, c_int64] + [_P] * 7 + [_P, c_size_t, _P, POINTER(c_void_p), c_int64, _P, _P]),
     "b200gs_ipc_alloc": (c_int32, [c_size_t, POINTER(c_void_p), ctypes.c_char_p]),
     "b200gs_ipc_open": (c_int32, [ctypes.c_char_p, POINTER(c_void_p)]),
     "b200gs_ipc_close": (c_int32, [c_void_p]),
     "b200gs_ipc_free": (c_int32, [c_void_p]),
     "b200gs_pack_rows_workspace_bytes": (c_size_t, [c_int64]),
     "b200gs_pack_rows": (c_int32, [c_int64, c_int64, c_int64] + [_P] * 7 + [_P, c_size_t, _P, _P, _P, _P]),
-    "b200gs_unpack_rows_grad": (c_int32, [c_int64] + [_P] * 9 + [_P]),
     "b200gs_bin_count_rows": (c_int32, [c_int32, c_int32, c_int32, c_int64, _P, c_int32, _P, c_size_t, _P, _P, c_int32, _P, _P, c_int64]),
     "b200gs_project_pack_workspace_bytes": (c_size_t, [c_int32, c_int64]),
     "b200gs_project_pack_multi": (c_int32, [POINTER(B200gsView), c_int32, c_int64] + [_P] * 6 + [c_int32] + [_P] * 4 + [POINTER(c_void_p), c_int64, _P, c_size_t, _P, _P]),

@@ -41,7 +41,7 @@ using namespace b200gs;
 extern "C" {
 
 const char* b200gs_last_error(void) { return g_error; }
-int b200gs_version(void) { return 220; }
+int b200gs_version(void) { return 230; }
 int64_t b200gs_launch_count(void) { return (int64_t)g_launches.load(std::memory_order_relaxed); }
 
 int b200gs_project_fwd(const B200gsView* view, int64_t n, const float* means, const float* scales, const float* quats,
@@ -107,25 +107,6 @@ int b200gs_project_fwd_rows(const B200gsView* view, int64_t n, const float* mean
     }
     return launch_project_fwd_raw(*view, n, means, log_scales, raw_quats, opacity_logits, shs_dc, shs_rest, anti_aliased, nullptr, nullptr,
                                   radii, nullptr, nullptr, tiles, nullptr, nullptr, clamped, nullptr, (cudaStream_t)stream, rows);
-}
-
-int b200gs_project_bwd_raw(const B200gsView* view, int64_t n, const float* means, const float* log_scales, const float* raw_quats,
-                           const float* opacity_logits, const float* shs_dc, const float* shs_rest, int32_t anti_aliased,
-                           const int32_t* radii, const uint8_t* clamped, const float* v_xy, const float* v_depth,
-                           const float* v_conic, const float* v_rgb, const float* v_opacity, float* v_means, float* v_log_scales,
-                           float* v_raw_quats, float* v_opacity_logits, float* v_shs_dc, float* v_shs_rest, void* stream) {
-    int rc = check_view(view, true);
-    if (rc) return rc;
-    B200GS_CHECK_ARG(n >= 0, "n < 0");
-    if (n > 0) {
-        B200GS_CHECK_ARG(means && log_scales && raw_quats && opacity_logits && shs_dc && radii && clamped, "NULL input pointer");
-        B200GS_CHECK_ARG(view->sh_stride == 1 || (shs_rest && v_shs_rest), "shs_rest / v_shs_rest required when sh_stride > 1");
-        B200GS_CHECK_ARG(v_xy && v_conic && v_rgb && v_opacity, "NULL cotangent pointer");
-        B200GS_CHECK_ARG(v_means && v_log_scales && v_raw_quats && v_opacity_logits && v_shs_dc, "NULL output pointer");
-    }
-    return launch_project_bwd_raw(*view, n, means, log_scales, raw_quats, opacity_logits, shs_dc, shs_rest, anti_aliased, radii,
-                                  clamped, v_xy, v_depth, v_conic, nullptr, v_rgb, v_opacity, v_means, v_log_scales, v_raw_quats,
-                                  v_opacity_logits, v_shs_dc, v_shs_rest, (cudaStream_t)stream);
 }
 
 int b200gs_project_bwd_rows(const B200gsView* view, int64_t n, const float* means, const float* log_scales, const float* raw_quats,
@@ -221,20 +202,6 @@ int b200gs_project_bwd_rows_multi(const B200gsView* views, int32_t n_views, int6
     return launch_project_bwd_multi(views, n_views, n, means, log_scales, raw_quats, opacity_logits, shs_dc, shs_rest, anti_aliased, radii, clamped,
                                     row_index, v_rows, v_means, v_log_scales, v_raw_quats, v_opacity_logits, v_shs_dc, v_shs_rest,
                                     (cudaStream_t)stream);
-}
-
-int b200gs_pack_rows_peer(int64_t n, int64_t segment_len, int64_t segment_cap, const float* xy, const float* depth, const float* conic,
-                          const float* comp, const float* opacity, const float* rgb, const int32_t* radii, void* workspace, size_t workspace_bytes,
-                          int32_t* row_index, float* const* peer_rows, int64_t peer_block, int64_t* d_count, void* stream) {
-    B200GS_CHECK_ARG(n >= 0 && segment_len > 0 && segment_cap > 0 && peer_block >= 0, "bad sizes");
-    B200GS_CHECK_ARG(peer_rows != nullptr && d_count != nullptr, "peer_rows / d_count must not be NULL");
-    if (n > 0) {
-        B200GS_CHECK_ARG(xy && depth && conic && opacity && rgb && radii && row_index && workspace, "NULL pointer");
-        B200GS_CHECK_ARG(workspace_bytes >= pack_rows_workspace_bytes(n), "workspace too small");
-        for (int64_t j = 0; j < (n + segment_len - 1) / segment_len; ++j) B200GS_CHECK_ARG(j >= B200GS_MAX_VIEWS || peer_rows[j] != nullptr, "NULL peer buffer");
-    }
-    return pack_rows(n, segment_len, segment_cap, xy, depth, conic, comp, opacity, rgb, radii, workspace, workspace_bytes, row_index, nullptr,
-                     d_count, (cudaStream_t)stream, peer_rows, peer_block);
 }
 
 int b200gs_ipc_alloc(size_t bytes, void** dev_ptr, unsigned char* handle64) {
@@ -380,19 +347,6 @@ int b200gs_blend_bwd(int32_t mode, int32_t width, int32_t height, int32_t channe
                             v_opacity, v_colors, v_xy_abs, (cudaStream_t)stream);
 }
 
-int b200gs_blend_bwd_to_rows(int32_t mode, int32_t width, int32_t height, const int32_t* tile_ranges, const int32_t* sorted_ids,
-                             const float* xy, const float* conic, const float* opacity, const float* colors, const float* bg,
-                             const float* final_T, const int32_t* n_contrib, const float* v_image, int64_t pix_stride, int64_t ch_stride,
-                             const float* v_alpha, float xy_scale_x, float xy_scale_y, float* v_rows, float* v_xy_abs, void* stream) {
-    B200GS_CHECK_ARG(mode == B200GS_MODE_VANILLA || mode == B200GS_MODE_GSPLAT, "bad mode");
-    B200GS_CHECK_ARG(width > 0 && height > 0, "bad size");
-    B200GS_CHECK_ARG(tile_ranges && final_T && n_contrib && v_image, "NULL input pointer");
-    B200GS_CHECK_ARG(v_rows != nullptr && (reinterpret_cast<uintptr_t>(v_rows) & 15) == 0, "v_rows must be a 16-byte aligned [n,12] buffer");
-    return launch_blend_bwd(mode, width, height, 3, tile_ranges, sorted_ids, 0, xy, conic, opacity, colors, bg, final_T, n_contrib, v_image,
-                            pix_stride, ch_stride, v_alpha, xy_scale_x, xy_scale_y, v_rows + B200GS_ROW_XY, v_rows + B200GS_ROW_CONIC,
-                            v_rows + B200GS_ROW_OPACITY, v_rows + B200GS_ROW_RGB, v_xy_abs, (cudaStream_t)stream, B200GS_ROW_FLOATS);
-}
-
 int b200gs_publish_i64(const int64_t* d_values, int64_t* host_values, int32_t n, void* stream) {
     B200GS_CHECK_ARG(d_values && host_values && n > 0, "bad argument");
     return publish_i64(d_values, host_values, n, (cudaStream_t)stream);
@@ -432,13 +386,6 @@ int b200gs_pack_rows(int64_t n, int64_t segment_len, int64_t segment_cap, const 
     B200GS_CHECK_ARG(n == 0 || workspace_bytes >= pack_rows_workspace_bytes(n), "workspace too small");
     return pack_rows(n, segment_len, segment_cap, xy, depth, conic, comp, opacity, rgb, radii, workspace, workspace_bytes, row_index, rows,
                      d_count, (cudaStream_t)stream);
-}
-
-int b200gs_unpack_rows_grad(int64_t n, const int32_t* radii, const int32_t* offsets, const float* v_rows, float* v_xy, float* v_depth,
-                            float* v_conic, float* v_comp, float* v_opacity, float* v_rgb, void* stream) {
-    B200GS_CHECK_ARG(n >= 0, "bad n");
-    B200GS_CHECK_ARG(n == 0 || (radii && offsets && v_xy && v_depth && v_conic && v_opacity && v_rgb), "NULL pointer");
-    return unpack_rows_grad(n, radii, offsets, v_rows, v_xy, v_depth, v_conic, v_comp, v_opacity, v_rgb, (cudaStream_t)stream);
 }
 
 int b200gs_bin_count_rows(int32_t mode, int32_t width, int32_t height, int64_t n, const float* rows, int32_t cull, void* workspace,

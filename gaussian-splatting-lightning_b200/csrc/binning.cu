@@ -1160,15 +1160,7 @@ __global__ void __launch_bounds__(256) visible_scan_kernel(int64_t n, const int3
 // rows past the capacity are dropped and reported through d_count[j] = visible entries of segment j (the caller compares
 // with seg_cap); unused rows of a block are zero-filled (radius 0 = culled for the binning that reads them in place).
 // row_index[i] is what the backward uses to find entry i's gradient row.
-// Peer mode (peers.p[seg] != NULL, segmented layout only): the row is not staged locally but stored STRAIGHT into the receive
-// buffer of the rank that owns camera `seg` — a peer GPU's memory mapped over NVLink — at row peer_block + k of it (peer_block
-// = this rank's block there): the projection's output reaches its consumer in one hop, no send buffer, no NCCL copy.
-struct PeerRows {
-    float* p[B200GS_MAX_VIEWS];
-};
-
-__global__ void __launch_bounds__(256) pack_rows_kernel(int64_t n, int64_t seg_len, int64_t seg_cap, const PeerRows peers, int64_t peer_block,
-                                                        const float2* __restrict__ xy,
+__global__ void __launch_bounds__(256) pack_rows_kernel(int64_t n, int64_t seg_len, int64_t seg_cap, const float2* __restrict__ xy,
                                                         const float* __restrict__ depth, const float* __restrict__ conic,
                                                         const float* __restrict__ comp, const float* __restrict__ opacity,
                                                         const float* __restrict__ rgb, const int32_t* __restrict__ radii,
@@ -1189,11 +1181,6 @@ __global__ void __launch_bounds__(256) pack_rows_kernel(int64_t n, int64_t seg_l
     row_index[i] = (int32_t)o;
     if (r <= 0 || o < 0) return;
     float4* out = reinterpret_cast<float4*>(rows + o * B200GS_ROW_FLOATS);
-    if (seg_cap > 0) {
-        const int64_t seg = i / seg_len;
-        if (seg < B200GS_MAX_VIEWS && peers.p[seg] != nullptr)
-            out = reinterpret_cast<float4*>(peers.p[seg] + (peer_block + (o - seg * seg_cap)) * B200GS_ROW_FLOATS);
-    }
     const float2 p = xy[i];
     out[0] = make_float4(p.x, p.y, depth[i], conic[3 * i]);
     out[1] = make_float4(conic[3 * i + 1], conic[3 * i + 2], comp ? comp[i] : 1.0f, opacity[i]);
@@ -1201,35 +1188,13 @@ __global__ void __launch_bounds__(256) pack_rows_kernel(int64_t n, int64_t seg_l
 }
 
 // zero the unused tail of every fixed-size block
-__global__ void __launch_bounds__(256) pad_rows_kernel(int64_t segments, int64_t seg_cap, const PeerRows peers, int64_t peer_block,
-                                                       const int64_t* __restrict__ d_count, float* __restrict__ rows) {
+__global__ void __launch_bounds__(256) pad_rows_kernel(int64_t segments, int64_t seg_cap, const int64_t* __restrict__ d_count,
+                                                       float* __restrict__ rows) {
     const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;    // one float4 per thread, 3 per row
     if (i >= segments * seg_cap * 3) return;
     const int64_t row = i / 3, seg = row / seg_cap, k = row - seg * seg_cap;
     if (k < d_count[seg]) return;
-    float4* dst = reinterpret_cast<float4*>(rows) + i;
-    if (seg < B200GS_MAX_VIEWS && peers.p[seg] != nullptr) dst = reinterpret_cast<float4*>(peers.p[seg] + (peer_block + k) * B200GS_ROW_FLOATS) + (i - row * 3);
-    *dst = make_float4(0.f, 0.f, 0.f, 0.f);
-}
-
-__global__ void __launch_bounds__(256) unpack_rows_grad_kernel(int64_t n, const int32_t* __restrict__ radii,
-                                                               const int32_t* __restrict__ offsets, const float* __restrict__ v_rows,
-                                                               float2* __restrict__ v_xy, float* __restrict__ v_depth,
-                                                               float* __restrict__ v_conic, float* __restrict__ v_comp,
-                                                               float* __restrict__ v_opacity, float* __restrict__ v_rgb) {
-    const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    float4 a = make_float4(0.f, 0.f, 0.f, 0.f), b = a, c = a;
-    if (radii[i] > 0) {
-        const float4* in = reinterpret_cast<const float4*>(v_rows + int64_t(offsets[i]) * B200GS_ROW_FLOATS);
-        a = in[0]; b = in[1]; c = in[2];
-    }
-    v_xy[i] = make_float2(a.x, a.y);
-    v_depth[i] = a.z;
-    v_conic[3 * i] = a.w; v_conic[3 * i + 1] = b.x; v_conic[3 * i + 2] = b.y;
-    if (v_comp) v_comp[i] = b.z;
-    v_opacity[i] = b.w;
-    v_rgb[3 * i] = c.x; v_rgb[3 * i + 1] = c.y; v_rgb[3 * i + 2] = c.z;
+    reinterpret_cast<float4*>(rows)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
 }
 
 }  // namespace
@@ -1240,16 +1205,8 @@ size_t pack_rows_workspace_bytes(int64_t n) { return pack_scan_state_bytes(n) + 
 
 int pack_rows(int64_t n, int64_t seg_len, int64_t seg_cap, const float* xy, const float* depth, const float* conic, const float* comp,
               const float* opacity, const float* rgb, const int32_t* radii, void* ws, size_t ws_bytes, int32_t* row_index, float* rows,
-              int64_t* d_count, cudaStream_t s, float* const* peer_rows, int64_t peer_block) {
+              int64_t* d_count, cudaStream_t s) {
     const int64_t segments = seg_cap > 0 ? div_up64(n, seg_len) : 1;
-    PeerRows peers{};
-    if (peer_rows != nullptr) {
-        if (seg_cap <= 0 || segments > B200GS_MAX_VIEWS) {
-            set_error("pack_rows: peer mode needs the segmented layout with at most %d segments", B200GS_MAX_VIEWS);
-            return B200GS_EINVAL;
-        }
-        for (int64_t j = 0; j < segments; ++j) peers.p[j] = peer_rows[j];
-    }
     if (n == 0) {
         B200GS_CUDA(cudaMemsetAsync(d_count, 0, sizeof(int64_t) * (size_t)segments, s));
         return B200GS_OK;
@@ -1262,22 +1219,13 @@ int pack_rows(int64_t n, int64_t seg_len, int64_t seg_cap, const float* xy, cons
     B200GS_CUDA(cudaMemsetAsync(ws, 0, state_bytes, s));
     visible_scan_kernel<<<(unsigned)div_up64(n, 256 * VS_ITEMS), 256, 0, s>>>(n, radii, scan, ticket, state);
     B200GS_LAUNCH_CHECK();
-    pack_rows_kernel<<<(unsigned)div_up64(n, 256), 256, 0, s>>>(n, seg_cap > 0 ? seg_len : n, seg_cap, peers, peer_block, (const float2*)xy, depth,
+    pack_rows_kernel<<<(unsigned)div_up64(n, 256), 256, 0, s>>>(n, seg_cap > 0 ? seg_len : n, seg_cap, (const float2*)xy, depth,
                                                                conic, comp, opacity, rgb, radii, scan, row_index, rows, d_count);
     B200GS_LAUNCH_CHECK();
     if (seg_cap > 0) {
-        pad_rows_kernel<<<(unsigned)div_up64(segments * seg_cap * 3, 256), 256, 0, s>>>(segments, seg_cap, peers, peer_block, d_count, rows);
+        pad_rows_kernel<<<(unsigned)div_up64(segments * seg_cap * 3, 256), 256, 0, s>>>(segments, seg_cap, d_count, rows);
         B200GS_LAUNCH_CHECK();
     }
-    return B200GS_OK;
-}
-
-int unpack_rows_grad(int64_t n, const int32_t* radii, const int32_t* offsets, const float* v_rows, float* v_xy, float* v_depth,
-                     float* v_conic, float* v_comp, float* v_opacity, float* v_rgb, cudaStream_t s) {
-    if (n == 0) return B200GS_OK;
-    unpack_rows_grad_kernel<<<(unsigned)div_up64(n, 256), 256, 0, s>>>(n, radii, offsets, v_rows, (float2*)v_xy, v_depth, v_conic, v_comp,
-                                                                      v_opacity, v_rgb);
-    B200GS_LAUNCH_CHECK();
     return B200GS_OK;
 }
 

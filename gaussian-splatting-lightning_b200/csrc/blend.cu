@@ -19,8 +19,6 @@
 // consecutive list entries and keeps their 9 partial derivatives in registers; the warp then reduces them with a
 // reduce-SCATTER butterfly (halving exchanges: RB -> RB/2 -> ... -> 1 value per lane) and one lane per splat issues
 // the atomics: 32x fewer L2 atomics than the reference's per-pixel atomicAdd.
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace b200gs {
@@ -113,12 +111,8 @@ __device__ __forceinline__ int build_list(const unsigned char* __restrict__ s_ma
     return n;
 }
 
-#ifndef B200GS_FWD_MINBLOCKS
-#define B200GS_FWD_MINBLOCKS 1
-#endif
-
 template <int CH, bool GSPLAT>
-__global__ void __launch_bounds__(BLOCK_PIX, B200GS_FWD_MINBLOCKS) blend_fwd_kernel(int width, int height, int grid_x, const int2* __restrict__ ranges,
+__global__ void __launch_bounds__(BLOCK_PIX, 1) blend_fwd_kernel(int width, int height, int grid_x, const int2* __restrict__ ranges,
                                                               const int32_t* __restrict__ ids, const SplatStrides st, const float* __restrict__ xy,
                                                               const float* __restrict__ conic, const float* __restrict__ opacity,
                                                               const float* __restrict__ colors, const float* __restrict__ bg,
@@ -638,13 +632,10 @@ int fwd_dispatch(int mode, int width, int height, const int32_t* ranges, const i
     //   first version of the asynchronous kernel (81 registers = 2 blocks per SM)            0.308-0.310 ms   vs synchronous 0.281-0.290 ms
     //   asynchronous kernel capped at 80 registers (3 blocks per SM), [n,12] rows (3 x 16 B)  0.277 ms         vs synchronous 0.290 ms
     // so the asynchronous staging is the default for the row layout (what the fused renderers and the sharded renderer use) and for the
-    // has_hit_any_pixels variant; the separate-array layout (eight 4/8-byte LDGSTS per splat) stays synchronous.
-    // B200GS_FWD_ASYNC=1 / =0 forces one or the other everywhere.
-    static const int async_env = []() { const char* e = getenv("B200GS_FWD_ASYNC"); return (e && e[0] == '1') ? 1 : (e && e[0] == '0') ? 0 : -1; }();
+    // has_hit_any_pixels variant; the separate-array layout (eight 4/8-byte LDGSTS per splat) stays synchronous (DESIGN.md §5.4).
     // the row layout is [x, y, depth, A, B, C, comp, opacity, r, g, b, radius] (include/b200gs.h); 16-byte copies need 16-byte aligned rows
     const bool rows16 = row_stride == 12 && CH == 3 && conic == xy + 3 && opacity == xy + 7 && colors == xy + 8 && (reinterpret_cast<uintptr_t>(xy) & 15) == 0;
-    const bool use_async = async_env == 1 || (async_env == -1 && rows16);
-    if (use_async || hit_any != nullptr) {
+    if (rows16 || hit_any != nullptr) {
 #define B200GS_FWD_ARGS width, height, gx, (const int2*)ranges, ids, st, xy, conic, opacity, colors, bg, image, ps, cs, final_T, n_contrib, alpha, hit_any
 #define B200GS_FWD_LAUNCH(G, R)                                                                                                   \
     do {                                                                                                                           \
@@ -678,14 +669,14 @@ int fwd_dispatch(int mode, int width, int height, const int32_t* ranges, const i
 template <int CH>
 int bwd_dispatch(int mode, int width, int height, const int32_t* ranges, const int32_t* ids, int row_stride, const float* xy, const float* conic,
                  const float* opacity, const float* colors, const float* bg, const float* final_T, const int32_t* n_contrib,
-                 const float* v_image, int64_t ps, int64_t cs, const float* v_alpha, float sx, float sy, int out_row_stride, float* v_xy,
+                 const float* v_image, int64_t ps, int64_t cs, const float* v_alpha, float sx, float sy, float* v_xy,
                  float* v_conic, float* v_opacity, float* v_colors, float* v_xy_abs, cudaStream_t s) {
     const int gx = div_up(width, TILE), gy = div_up(height, TILE);
     dim3 grid(gx * gy);
     const SplatStrides st = row_stride > 0 ? SplatStrides{row_stride, row_stride, row_stride, row_stride} : SplatStrides{2, 3, 1, CH};
-    const SplatStrides so = out_row_stride > 0 ? SplatStrides{out_row_stride, out_row_stride, out_row_stride, out_row_stride} : SplatStrides{2, 3, 1, CH};
+    const SplatStrides so = st;   // the gradients have the layout of the inputs
     // gradient outputs that are the columns of one 16-byte aligned [n,12] row buffer leave as 128-bit reductions
-    const bool vrows = CH == 3 && out_row_stride == B200GS_ROW_FLOATS && v_conic == v_xy + B200GS_ROW_CONIC && v_opacity == v_xy + B200GS_ROW_OPACITY &&
+    const bool vrows = CH == 3 && row_stride == B200GS_ROW_FLOATS && v_conic == v_xy + B200GS_ROW_CONIC && v_opacity == v_xy + B200GS_ROW_OPACITY &&
                        v_colors == v_xy + B200GS_ROW_RGB && (reinterpret_cast<uintptr_t>(v_xy) & 15) == 0;
 #define B200GS_BWD_ARGS width, height, gx, (const int2*)ranges, ids, st, so, xy, conic, opacity, colors, bg, final_T, n_contrib, \
                         v_image, ps, cs, v_alpha, sx, sy, v_xy, v_conic, v_opacity, v_colors, v_xy_abs
@@ -702,8 +693,6 @@ int bwd_dispatch(int mode, int width, int height, const int32_t* ranges, const i
         if constexpr (CH == 3) {
             set((const void*)blend_bwd_tr_kernel<CH, true, false, true>, sizeof(TrSmem<false>));
             set((const void*)blend_bwd_tr_kernel<CH, false, false, true>, sizeof(TrSmem<false>));
-            set((const void*)blend_bwd_tr_kernel<CH, true, true, true>, sizeof(TrSmem<true>));
-            set((const void*)blend_bwd_tr_kernel<CH, false, true, true>, sizeof(TrSmem<true>));
         }
         return e;
     }();
@@ -714,9 +703,9 @@ int bwd_dispatch(int mode, int width, int height, const int32_t* ranges, const i
 #define B200GS_BWD_LAUNCH(G, A, V) blend_bwd_tr_kernel<CH, G, A, V><<<grid, BLOCK_PIX, sizeof(TrSmem<A>), s>>>(B200GS_BWD_ARGS)
     const bool gs = mode == B200GS_MODE_GSPLAT, ab = v_xy_abs != nullptr;
     if (vrows) {
-        if constexpr (CH == 3) {
-            if (gs) { if (ab) B200GS_BWD_LAUNCH(true, true, true); else B200GS_BWD_LAUNCH(true, false, true); }
-            else    { if (ab) B200GS_BWD_LAUNCH(false, true, true); else B200GS_BWD_LAUNCH(false, false, true); }
+        if constexpr (CH == 3) {   // the row entry point has no absgrad output
+            if (gs) B200GS_BWD_LAUNCH(true, false, true);
+            else B200GS_BWD_LAUNCH(false, false, true);
         }
     } else {
         if (gs) { if (ab) B200GS_BWD_LAUNCH(true, true, false); else B200GS_BWD_LAUNCH(true, false, false); }
@@ -748,10 +737,9 @@ int launch_blend_bwd(int mode, int width, int height, int channels, const int32_
                      const float* conic, const float* opacity, const float* colors, const float* bg, const float* final_T,
                      const int32_t* n_contrib, const float* v_image, int64_t pix_stride, int64_t ch_stride, const float* v_alpha,
                      float sx, float sy, float* v_xy, float* v_conic, float* v_opacity, float* v_colors, float* v_xy_abs,
-                     cudaStream_t s, int out_row_stride) {
-    if (out_row_stride < 0) out_row_stride = row_stride;
+                     cudaStream_t s) {
 #define B200GS_BWD_CALL(C) bwd_dispatch<C>(mode, width, height, ranges, ids, row_stride, xy, conic, opacity, colors, bg, final_T, n_contrib, v_image, \
-                                           pix_stride, ch_stride, v_alpha, sx, sy, out_row_stride, v_xy, v_conic, v_opacity, v_colors, v_xy_abs, s)
+                                           pix_stride, ch_stride, v_alpha, sx, sy, v_xy, v_conic, v_opacity, v_colors, v_xy_abs, s)
     switch (channels) {
         case 1: return B200GS_BWD_CALL(1);
         case 2: return B200GS_BWD_CALL(2);

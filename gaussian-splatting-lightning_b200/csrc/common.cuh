@@ -115,9 +115,7 @@ int publish_i64(const int64_t* d_values, int64_t* host_values, int n, cudaStream
 size_t pack_rows_workspace_bytes(int64_t n);
 int pack_rows(int64_t n, int64_t seg_len, int64_t seg_cap, const float* xy, const float* depth, const float* conic, const float* comp,
               const float* opacity, const float* rgb, const int32_t* radii, void* ws, size_t ws_bytes, int32_t* row_index, float* rows,
-              int64_t* d_count, cudaStream_t s, float* const* peer_rows = nullptr, int64_t peer_block = 0);
-int unpack_rows_grad(int64_t n, const int32_t* radii, const int32_t* offsets, const float* v_rows, float* v_xy, float* v_depth,
-                     float* v_conic, float* v_comp, float* v_opacity, float* v_rgb, cudaStream_t s);
+              int64_t* d_count, cudaStream_t s);
 int bin_sort(int mode, int width, int height, int64_t n, int cull, int64_t max_coarse, int64_t max_pairs, int64_t* d_counts,
              const void* ws_a, void* ws_b, size_t ws_b_bytes, int32_t* sorted_ids, int32_t* tile_ranges, int64_t* host_counts,
              int sync_host, cudaStream_t s);
@@ -143,6 +141,6 @@ int launch_blend_bwd(int mode, int width, int height, int channels, const int32_
                      int row_stride, const float* xy, const float* conic, const float* opacity, const float* colors, const float* bg,
                      const float* final_T, const int32_t* n_contrib, const float* v_image, int64_t pix_stride,
                      int64_t ch_stride, const float* v_alpha, float sx, float sy, float* v_xy, float* v_conic,
-                     float* v_opacity, float* v_colors, float* v_xy_abs, cudaStream_t s, int out_row_stride = -1);
+                     float* v_opacity, float* v_colors, float* v_xy_abs, cudaStream_t s);
 
 }  // namespace b200gs

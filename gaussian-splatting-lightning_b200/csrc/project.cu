@@ -8,8 +8,6 @@
 //
 // HBM-bound: per visible Gaussian 268 B fwd / 552 B bwd at SH degree 3.  SH coefficients are streamed with
 // 128-bit read-only loads (ld.global.nc), outputs written with 64/128-bit stores where the layout allows.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "onesweep.cuh"
 
@@ -266,7 +264,6 @@ struct RawIO {
     const float* v_rows;
     const int32_t* row_offsets;
     int accumulate;
-    int prefetch_sh;         // K1: L2 prefetch of the SH row of every Gaussian in front of the camera, issued before the fp64 geometry
     float* v_mean2d;         // K8 (rows path, optional): [n, v_mean2d_cols] <- (dL/dmean2D.x, .y[, 0]) of every Gaussian, zeros for culled ones:
     int v_mean2d_cols;       // the `viewspace_points.grad` of the renderer contract, written here instead of by a fill + strided copy
 };
@@ -432,14 +429,6 @@ __device__ __forceinline__ void sh_color_one(const B200gsView& v, const float* p
     if (bc < 0.f) { bc = 0.f; cl |= 4; }
 }
 
-// L2 prefetch of the first `floats` floats at `row` (one request per 64 bytes + the last word)
-__device__ __forceinline__ void prefetch_l2(const float* row, int floats) {
-    const char* r = reinterpret_cast<const char*>(row);
-    const int bytes = floats * 4;
-    for (int off = 0; off < bytes; off += 64) asm volatile("prefetch.global.L2 [%0];" ::"l"(r + off));
-    if (bytes > 0) asm volatile("prefetch.global.L2 [%0];" ::"l"(r + bytes - 4));
-}
-
 // rows_out (raw mode only): instead of the separate arrays, ONE [n,12] row per Gaussian (xy 0..1, depth 2, conic 3..5, compensation 6,
 // blend opacity 7, rgb 8..10, radius bits 11) — three 128-bit stores; the binning and the blend kernels read the rows in place (one
 // 48-byte record per splat instead of four separate sectors).  radii_out / clamped_out (what K8 needs) are still written.
@@ -455,17 +444,6 @@ __global__ void __launch_bounds__(256, 3) project_fwd_kernel(const __grid_consta
     const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const float p[3] = {__ldg(means + 3 * i), __ldg(means + 3 * i + 1), __ldg(means + 3 * i + 2)};
-    if (raw.prefetch_sh && shs != nullptr) {
-        // The SH row is only needed once the Gaussian is known to be visible, i.e. after ~150 dependent fp64 operations.  Opt-in
-        // (B200GS_K1_PREFETCH=1): everything in front of the camera gets its row pulled into L2 before the geometry.
-        const float* V = v.viewmatrix;
-        const float tz = p[0] * V[2] + p[1] * V[6] + p[2] * V[10] + V[14];
-        if (tz > 0.f) {
-            const int rw = (RAW ? v.sh_stride - 1 : v.sh_stride) * 3;
-            const int need = ((v.sh_degree + 1) * (v.sh_degree + 1) - (RAW ? 1 : 0)) * 3;
-            prefetch_l2((RAW ? raw.shs_rest : shs) + i * int64_t(rw), min(rw, need));
-        }
-    }
     double sc[3], q[4], inv_qn;
     load_scale_quat<RAW, double>(scales, quats, i, sc, q, &inv_qn);
     const ProjOut out{xy_out, depth_out, radii_out, conic_out, comp_out, tiles_out, cov3d_out, rgb_out, clamped_out};
@@ -514,10 +492,6 @@ __global__ void __launch_bounds__(256) project_fwd_multi_kernel(const __grid_con
     const float p[3] = {__ldg(means + 3 * i), __ldg(means + 3 * i + 1), __ldg(means + 3 * i + 2)};
     double sc[3], q[4], inv_qn;
     load_scale_quat<true, double>(scales, quats, i, sc, q, &inv_qn);
-    if (raw.prefetch_sh) {   // the SH row is needed after the whole camera loop: pull it into L2 now (B200GS_K1_PREFETCH=1)
-        const int deg0 = vp.v[0].sh_degree;
-        prefetch_l2(raw.shs_rest + i * int64_t(vp.v[0].sh_stride - 1) * 3, min((vp.v[0].sh_stride - 1) * 3, ((deg0 + 1) * (deg0 + 1) - 1) * 3));
-    }
     Proj<double> g3;
     gaussian_cov3d<double>(sc, q, vp.v[0].scale_modifier, g3);      // once per Gaussian; project_one_view per camera
     const ProjOut out{xy_out, depth_out, radii_out, conic_out, nullptr, nullptr, nullptr, rgb_out, clamped_out};
@@ -584,10 +558,6 @@ __global__ void __launch_bounds__(PACK_THREADS, (MC <= 16 ? 3 : 2)) project_pack
     if (live) {
         p[0] = __ldg(means + 3 * i); p[1] = __ldg(means + 3 * i + 1); p[2] = __ldg(means + 3 * i + 2);
         load_scale_quat<true, double>(scales, quats, i, sc, q, &inv_qn);
-        if (raw.prefetch_sh) {   // the SH row is needed after the whole camera loop: pull it into L2 now (B200GS_K1_PREFETCH=1)
-            const int deg0 = vp.v[0].sh_degree;
-            prefetch_l2(raw.shs_rest + i * int64_t(vp.v[0].sh_stride - 1) * 3, min((vp.v[0].sh_stride - 1) * 3, ((deg0 + 1) * (deg0 + 1) - 1) * 3));
-        }
     }
     Proj<double> g3;
     gaussian_cov3d<double>(sc, q, vp.v[0].scale_modifier, g3);      // once per Gaussian; project_one_view per camera
@@ -1185,11 +1155,6 @@ int launch_project_fwd(const B200gsView& v, int64_t n, const float* means, const
                                   rgb, clamped, nullptr, s, nullptr);
 }
 
-static bool sh_prefetch_enabled() {
-    static const bool on = []() { const char* e = getenv("B200GS_K1_PREFETCH"); return e && e[0] == '1'; }();
-    return on;
-}
-
 int launch_project_fwd_raw(const B200gsView& v, int64_t n, const float* means, const float* scales, const float* quats,
                            const float* opac_logits, const float* shs_dc, const float* shs_rest, int anti_aliased, float* xy,
                            float* depth, int32_t* radii, float* conic, float* comp, int32_t* tiles, float* cov3d, float* rgb,
@@ -1200,9 +1165,6 @@ int launch_project_fwd_raw(const B200gsView& v, int64_t n, const float* means, c
     const bool raw_mode = opac_out != nullptr || rows != nullptr;
     RawIO raw{opac_logits, shs_rest, opac_out, nullptr, nullptr, nullptr, anti_aliased, nullptr, nullptr, 0};
 #define B200GS_PF_ARGS v, raw, n, means, scales, quats, shs_dc, (float2*)xy, depth, radii, conic, comp, tiles, cov3d, rgb, clamped, rows
-    // L2 prefetch of the SH rows ahead of the fp64 geometry: measured 0.085 ms with, 0.079 ms without at 1 M / 1080p (the extra
-    // requests of the frustum-culled Gaussians cost more than the hidden latency returns): opt-in (B200GS_K1_PREFETCH=1)
-    raw.prefetch_sh = sh_prefetch_enabled() ? 1 : 0;
 #define B200GS_PF_LAUNCH(MC)                                                                                    \
     do {                                                                                                         \
         if (v.mode == B200GS_MODE_GSPLAT) {                                                                      \
@@ -1239,7 +1201,7 @@ int launch_project_bwd_raw(const B200gsView& v, int64_t n, const float* means, c
     const int threads = BWD_THREADS;
     const unsigned blocks = (unsigned)div_up64(n, threads);
     const bool raw_mode = v_opac_logit != nullptr;
-    RawIO raw{opac_logits, shs_rest, nullptr, v_opac, v_opac_logit, v_shs_rest, anti_aliased, v_rows, row_offsets, accumulate, 0, v_mean2d, v_mean2d_cols};
+    RawIO raw{opac_logits, shs_rest, nullptr, v_opac, v_opac_logit, v_shs_rest, anti_aliased, v_rows, row_offsets, accumulate, v_mean2d, v_mean2d_cols};
 #define B200GS_PB_ARGS v, raw, n, means, scales, quats, shs_dc, radii, clamped, (const float2*)v_xy, v_depth, v_conic, v_comp, v_rgb, \
                        v_means, v_scales, (float4*)v_quats, v_shs_dc
 #define B200GS_PB_LAUNCH(MC)                                                                                    \
@@ -1268,7 +1230,6 @@ int launch_project_fwd_multi(const B200gsView* views, int n_views, int64_t n, co
     for (int j = 0; j < n_views; ++j) vp.v[j] = views[j];
     for (int j = n_views; j < B200GS_MAX_VIEWS; ++j) vp.v[j] = views[0];
     RawIO raw{opac_logits, shs_rest, opac_out, nullptr, nullptr, nullptr, anti_aliased, nullptr, nullptr, 0};
-    raw.prefetch_sh = sh_prefetch_enabled() ? 1 : 0;
     if (views[0].sh_degree > 3)
         project_fwd_multi_kernel<25><<<(unsigned)div_up64(n, 256), 256, 0, s>>>(vp, n_views, raw, n, means, scales, quats, shs_dc, (float2*)xy, depth,
                                                                                 radii, conic, rgb, clamped);
@@ -1304,7 +1265,6 @@ int launch_project_pack_multi(const B200gsView* views, int n_views, int64_t n, c
         dst.p[j] = j < n_views ? dst_rows[j] : nullptr;
     }
     RawIO raw{opac_logits, shs_rest, nullptr, nullptr, nullptr, nullptr, anti_aliased, nullptr, nullptr, 0};
-    raw.prefetch_sh = sh_prefetch_enabled() ? 1 : 0;
     B200GS_CUDA(cudaMemsetAsync(workspace, 0, need, s));
     uint32_t* ticket = (uint32_t*)workspace;
     uint32_t* state = ticket + 64;

@@ -281,7 +281,7 @@ class PeerExchange:
     """Exchange buffers every rank of the box can address: each rank owns two receive buffers for splat rows (alternating by
     step) and one for gradient rows, `world * rows_per_block` rows of 12 floats each, allocated with cudaMalloc and mapped into
     the peers with CUDA IPC (b200gs_ipc_*).  Producers store rows straight into the owner's buffer from their pack kernel
-    (b200gs_pack_rows_peer) and consumers pull gradient rows straight out of the owner's buffer in K8 — NVLink loads/stores from
+    (b200gs_project_pack_multi) and consumers pull gradient rows straight out of the owner's buffer in K8 — NVLink loads/stores from
     our own kernels, no all-to-all.  All methods are collective."""
 
     def __init__(self, group, device):

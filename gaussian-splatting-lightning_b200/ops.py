@@ -180,7 +180,6 @@ _host_counts_pool = []  # pinned int64[8] buffers: [0:4] phase A's copy of the c
 _last_total = {}       # key -> (coarse pairs, rect pairs) of the previous view: sizes the next view's buffers in lazy mode
 _state_lock = threading.RLock()   # the two process-wide structures above are shared by every thread that renders (trainer + viewer threads)
 
-TILE_CULLING = True    # exact (tile, splat) culling in K3; False reproduces the reference's full 3-sigma-rect pair list
 LAZY_SLACK = 1.15      # lazy mode: capacity = slack x previous count
 
 
@@ -242,7 +241,7 @@ def bin_gaussians(mode: int, width: int, height: int, xy: torch.Tensor, depth: t
     call Binning.resolve() once the rest of the forward is enqueued — it returns False in the rare case a capacity was
     exceeded and the forward has to be redone with lazy=False."""
     L = lib()
-    if not TILE_CULLING or conic is None or opacity is None:
+    if conic is None or opacity is None:
         conic = opacity = None
     n = xy.shape[0]
 
@@ -454,49 +453,8 @@ def rasterize_vanilla(means3D, means2D, shs, colors_precomp, opacities, scales, 
 
 
 # ----------------------------------------------------------------------------------------------------------------------
-# vanilla, activations fused: the same node fed with the model's RAW parameter tensors (b200gs_project_*_raw)
+# vanilla, activations fused: the same node fed with the model's RAW parameter tensors (b200gs_project_*_rows)
 # ----------------------------------------------------------------------------------------------------------------------
-def project_forward_raw(view: B200gsView, means, log_scales, raw_quats, opac_logits, shs_dc, shs_rest, anti_aliased=False,
-                        want_comp=False):
-    L = lib()
-    n = means.shape[0]
-    dev = means.device
-    xy = torch.empty(n, 2, dtype=torch.float32, device=dev)
-    depth = torch.empty(n, dtype=torch.float32, device=dev)
-    radii = torch.empty(n, dtype=torch.int32, device=dev)
-    conic = torch.empty(n, 3, dtype=torch.float32, device=dev)
-    tiles = torch.empty(n, dtype=torch.int32, device=dev)
-    comp = torch.empty(n, dtype=torch.float32, device=dev) if want_comp else None
-    rgb = torch.empty(n, 3, dtype=torch.float32, device=dev)
-    clamped = torch.empty(n, dtype=torch.uint8, device=dev)
-    opac = torch.empty(n, dtype=torch.float32, device=dev)
-    with _stage("project_fwd"):
-        check(L.b200gs_project_fwd_raw(ctypes.byref(view), n, ptr(means), ptr(log_scales), ptr(raw_quats), ptr(opac_logits),
-                                       ptr(shs_dc), ptr(shs_rest), int(bool(anti_aliased)), ptr(xy), ptr(depth), ptr(radii),
-                                       ptr(conic), ptr(comp), ptr(tiles), ptr(rgb), ptr(clamped), ptr(opac), _stream()),
-              "b200gs_project_fwd_raw")
-    return xy, depth, radii, conic, comp, tiles, rgb, clamped, opac
-
-
-def project_backward_raw(view: B200gsView, means, log_scales, raw_quats, opac_logits, shs_dc, shs_rest, anti_aliased, radii,
-                         clamped, v_xy, v_depth, v_conic, v_rgb, v_opac):
-    L = lib()
-    n = means.shape[0]
-    dev = means.device
-    v_means = torch.empty(n, 3, dtype=torch.float32, device=dev)
-    v_ls = torch.empty(n, 3, dtype=torch.float32, device=dev)
-    v_q = torch.empty(n, 4, dtype=torch.float32, device=dev)
-    v_ol = torch.empty(n, dtype=torch.float32, device=dev)
-    v_dc = torch.empty_like(shs_dc)
-    v_rest = torch.empty_like(shs_rest)
-    with _stage("project_bwd"):
-        check(L.b200gs_project_bwd_raw(ctypes.byref(view), n, ptr(means), ptr(log_scales), ptr(raw_quats), ptr(opac_logits),
-                                       ptr(shs_dc), ptr(shs_rest), int(bool(anti_aliased)), ptr(radii), ptr(clamped), ptr(v_xy),
-                                       ptr(v_depth), ptr(v_conic), ptr(v_rgb), ptr(v_opac), ptr(v_means), ptr(v_ls), ptr(v_q),
-                                       ptr(v_ol), ptr(v_dc), ptr(v_rest), _stream()), "b200gs_project_bwd_raw")
-    return v_means, v_ls, v_q, v_ol, v_dc, v_rest
-
-
 class _RasterizeRaw(torch.autograd.Function):
     """The whole renderer step as ONE autograd node on the model's RAW parameters, either constant set: K1 (activations + SH fused)
     writes one [N,12] row per Gaussian, K2-K6 read the rows in place; backward: K7 accumulates [N,12] gradient rows (128-bit
@@ -609,45 +567,6 @@ class _ProjectGaussians(torch.autograd.Function):
         v_means, v_scales, v_quats, _ = project_backward(ctx.view, means3d, scales, quats, None, radii, None, z(v_xy, (n, 2)),
                                                          z(v_depth, (n,)), z(v_conic, (n, 3)), z(v_comp, (n,)), None)
         return v_means, v_scales, v_quats, None
-
-
-class _ProjectGaussiansRaw(torch.autograd.Function):
-    """gsplat-mode K1 / K8 on the model's RAW parameters (activations, compensation-scaled opacity and SH colours fused):
-    -> xys, depths, radii, conics, tiles, opacity_for_blend [N], rgbs [N,3].  `xys` stays a graph tensor so the
-    renderer's ``viewspace_points.retain_grad()`` contract holds."""
-
-    @staticmethod
-    def forward(ctx, means, log_scales, raw_quats, opac_logits, shs_dc, shs_rest, view: B200gsView, anti_aliased: bool):
-        means = _f32c(means, "means")
-        log_scales = _f32c(log_scales, "scales")
-        raw_quats = _f32c(raw_quats, "rotations")
-        ol = _f32c(opac_logits, "opacities").reshape(-1)
-        shs_dc = _f32c(shs_dc, "shs_dc")
-        shs_rest = _f32c(shs_rest, "shs_rest")
-        view = _copy_view(view, sh_stride=int(shs_dc.shape[1] + shs_rest.shape[1]))
-        xy, depth, radii, conic, _, tiles, rgb, clamped, opac = project_forward_raw(view, means, log_scales, raw_quats, ol, shs_dc, shs_rest,
-                                                                                  anti_aliased)
-        ctx.view, ctx.aa, ctx.opac_shape = view, bool(anti_aliased), tuple(opac_logits.shape)
-        ctx.save_for_backward(means, log_scales, raw_quats, ol, shs_dc, shs_rest, radii, clamped)
-        ctx.mark_non_differentiable(radii, tiles)
-        return xy, depth, radii, conic, tiles, opac, rgb
-
-    @staticmethod
-    def backward(ctx, v_xy, v_depth, _v_radii, v_conic, _v_tiles, v_opac, v_rgb):
-        means, log_scales, raw_quats, ol, shs_dc, shs_rest, radii, clamped = ctx.saved_tensors
-        n, dev = means.shape[0], means.device
-
-        def z(t, shape):
-            return torch.zeros(shape, dtype=torch.float32, device=dev) if t is None else _f32c(t, "grad")
-
-        v_means, v_ls, v_q, v_ol, v_dc, v_rest = project_backward_raw(
-            ctx.view, means, log_scales, raw_quats, ol, shs_dc, shs_rest, ctx.aa, radii, clamped, z(v_xy, (n, 2)),
-            None if v_depth is None else _f32c(v_depth, "grad"), z(v_conic, (n, 3)), z(v_rgb, (n, 3)), z(v_opac, (n,)))
-        return v_means, v_ls, v_q, v_ol.reshape(ctx.opac_shape), v_dc, v_rest, None, None
-
-
-def project_gaussians_raw(means, log_scales, raw_quats, opacity_logits, shs_dc, shs_rest, view: B200gsView, anti_aliased: bool = True):
-    return _ProjectGaussiansRaw.apply(means, log_scales, raw_quats, opacity_logits, shs_dc, shs_rest, view, anti_aliased)
 
 
 def project_gaussians(means3d, scales, glob_scale, quats, viewmat, fx, fy, cx, cy, img_height, img_width, block_width=16,

@@ -108,17 +108,11 @@ B200GS_API int b200gs_project_bwd(const B200gsView* view, int64_t n, const float
  * concatenation and their autograd backward from every training step.
  * fwd extra out: opacity_out[n] = the opacity the blend kernels consume (x compensation in gsplat mode when
  *     anti_aliased != 0; gsplat_renderer.py:81-83).
- * bwd extra in : v_opacity[n] = dL/d(opacity_out) from b200gs_blend_bwd; outputs are gradients w.r.t. the RAW tensors. */
+ * The matching K8 is b200gs_project_bwd_rows (below): gradients w.r.t. the RAW tensors, cotangents from gradient rows. */
 B200GS_API int b200gs_project_fwd_raw(const B200gsView* view, int64_t n, const float* means, const float* log_scales,
                            const float* raw_quats, const float* opacity_logits, const float* shs_dc, const float* shs_rest,
                            int32_t anti_aliased, float* xy, float* depth, int32_t* radii, float* conic, float* comp,
                            int32_t* tiles, float* rgb, uint8_t* clamped, float* opacity_out, void* stream);
-B200GS_API int b200gs_project_bwd_raw(const B200gsView* view, int64_t n, const float* means, const float* log_scales,
-                           const float* raw_quats, const float* opacity_logits, const float* shs_dc, const float* shs_rest,
-                           int32_t anti_aliased, const int32_t* radii, const uint8_t* clamped, const float* v_xy,
-                           const float* v_depth, const float* v_conic, const float* v_rgb, const float* v_opacity, float* v_means,
-                           float* v_log_scales, float* v_raw_quats, float* v_opacity_logits, float* v_shs_dc, float* v_shs_rest,
-                           void* stream);
 
 /* ---- per-Gaussian passes next to the renderer in a training step (SURVEY §8f rank 4) ---------------------------------------
  * b200gs_selective_adam: visibility-masked Adam step of one [rows, width] parameter tensor (gsplat.optimizers.SelectiveAdam /
@@ -223,15 +217,6 @@ B200GS_API int b200gs_blend_bwd(int32_t mode, int32_t width, int32_t height, int
                      float xy_scale_x, float xy_scale_y, float* v_xy, float* v_conic, float* v_opacity,
                      float* v_colors, float* v_xy_abs, void* stream);
 
-/* b200gs_blend_bwd_to_rows: K7 on separate input arrays (3 colour channels) accumulating into ONE zero-filled, 16-byte aligned
- *     gradient row buffer v_rows[n,12] (row layout below: xy 0..1, conic 3..5, opacity 7, rgb 8..10; the other columns stay 0): the
- *     nine sums of a (warp, splat) leave the SM as three 128-bit reductions instead of nine 32-bit atomics.  K8 consumes the rows
- *     directly (b200gs_project_bwd_rows with row_offsets = NULL: row i belongs to Gaussian i). */
-B200GS_API int b200gs_blend_bwd_to_rows(int32_t mode, int32_t width, int32_t height, const int32_t* tile_ranges, const int32_t* sorted_ids,
-                     const float* xy, const float* conic, const float* opacity, const float* colors, const float* bg,
-                     const float* final_T, const int32_t* n_contrib, const float* v_image, int64_t pix_stride, int64_t ch_stride,
-                     const float* v_alpha, float xy_scale_x, float xy_scale_y, float* v_rows, float* v_xy_abs, void* stream);
-
 /* ---- fused L1 + SSIM training loss on the rendered image (validated on B200: tests/test_gpu_loss.py) -------------------------
  * replaces  loss = (1-lambda) * l1_loss(image, gt) + lambda * (1 - ssim(image, gt))   (internal/metrics/vanilla_metrics.py:57-74,
  * internal/utils/ssim.py:17-63: 11-tap Gaussian window sigma 1.5, zero padding, C1 = 0.01^2, C2 = 0.03^2).  image/target [C,H,W].
@@ -254,12 +239,10 @@ B200GS_API int b200gs_loss_bwd(int32_t channels, int32_t width, int32_t height, 
  *     block rows[j*segment_cap, (j+1)*segment_cap) — the all-to-all then needs no size exchange (no host sync); unused
  *     rows are zero (radius 0: ignored by the binning that reads them in place); entries that do not fit are DROPPED
  *     (row_index -1) and d_count[j] <- visible entries of segment j, for the caller to compare with segment_cap.
- * b200gs_unpack_rows_grad: the backward of that gather: full-length per-Gaussian cotangents for b200gs_project_bwd*
- *     (zeros for culled Gaussians).
  * b200gs_bin_count_rows (then b200gs_bin_sort) / blend_fwd_rows / blend_bwd_rows: K2-K7 reading the rows IN PLACE (strided
  *     access, no split copies); blend_bwd_rows accumulates into a zero-filled [n,12] gradient row buffer that goes
  *     straight back through the all-to-all.  3 colour channels; cull != 0 enables exact tile culling. */
-#define B200GS_MAX_VIEWS 8      /* cameras per multi-view launch / destination ranks per peer-mode pack (one NVSwitch box) */
+#define B200GS_MAX_VIEWS 8      /* cameras per multi-view launch (one NVSwitch box) */
 #define B200GS_ROW_FLOATS 12
 #define B200GS_ROW_XY 0
 #define B200GS_ROW_DEPTH 2
@@ -302,7 +285,7 @@ B200GS_API int b200gs_project_fwd_raw_multi(const B200gsView* views, int32_t n_v
  *     pointers: block of block_rows rows in the receive buffer of the rank that owns camera j — peer memory over NVLink — or in a local
  *     send buffer); rows past block_rows are dropped.  d_count[j] = visible splats of camera j (compare with block_rows).  Kept locally
  *     for K8 and the renderer contract, camera-major ([j*n + i]): xy (mean2D), radii, clamped, row_index (j*block_rows + k, -1 = dropped).
- *     Replaces b200gs_project_fwd_raw_multi + b200gs_pack_rows(_peer) (gsplat_distributed_renderer.py:127-217: project, then all-to-all). */
+ *     Replaces b200gs_project_fwd_raw_multi + b200gs_pack_rows (gsplat_distributed_renderer.py:127-217: project, then all-to-all). */
 B200GS_API size_t b200gs_project_pack_workspace_bytes(int32_t n_views, int64_t n);
 B200GS_API int b200gs_project_pack_multi(const B200gsView* views, int32_t n_views, int64_t n, const float* means, const float* log_scales,
                                          const float* raw_quats, const float* opacity_logits, const float* shs_dc, const float* shs_rest,
@@ -314,16 +297,8 @@ B200GS_API int b200gs_project_bwd_rows_multi(const B200gsView* views, int32_t n_
                                              int32_t anti_aliased, const int32_t* radii, const uint8_t* clamped, const int32_t* row_index,
                                              const float* const* v_rows, float* v_means, float* v_log_scales, float* v_raw_quats,
                                              float* v_opacity_logits, float* v_shs_dc, float* v_shs_rest, void* stream);
-/* b200gs_pack_rows_peer: b200gs_pack_rows in the segmented layout, but segment j's rows (and the zero rows that pad its block) are
- *     stored straight into peer_rows[j] — the receive buffer of the rank that owns camera j, possibly a peer GPU's memory — at
- *     rows [peer_block, peer_block + segment_cap) of it; peer_rows is a HOST array of ceil(n/segment_len) device pointers.
- *     `rows` is unused then (may be NULL); row_index keeps the send-layout numbering j*segment_cap + k.
- * b200gs_ipc_alloc / _handle / _open / _close / _free: device buffers that peer processes of the same box can map (cudaMalloc +
+/* b200gs_ipc_alloc / _handle / _open / _close / _free: device buffers that peer processes of the same box can map (cudaMalloc +
  *     CUDA IPC): the exchange buffers of the sharded renderer.  handle = 64 bytes to pass to the peers by any host channel. */
-B200GS_API int b200gs_pack_rows_peer(int64_t n, int64_t segment_len, int64_t segment_cap, const float* xy, const float* depth,
-                                     const float* conic, const float* comp, const float* opacity, const float* rgb, const int32_t* radii,
-                                     void* workspace, size_t workspace_bytes, int32_t* row_index, float* const* peer_rows, int64_t peer_block,
-                                     int64_t* d_count, void* stream);
 B200GS_API int b200gs_ipc_alloc(size_t bytes, void** dev_ptr, unsigned char* handle64);
 B200GS_API int b200gs_ipc_open(const unsigned char* handle64, void** dev_ptr);
 B200GS_API int b200gs_ipc_close(void* dev_ptr);
@@ -332,8 +307,6 @@ B200GS_API size_t b200gs_pack_rows_workspace_bytes(int64_t n);
 B200GS_API int b200gs_pack_rows(int64_t n, int64_t segment_len, int64_t segment_cap, const float* xy, const float* depth,
                                 const float* conic, const float* comp, const float* opacity, const float* rgb, const int32_t* radii,
                                 void* workspace, size_t workspace_bytes, int32_t* row_index, float* rows, int64_t* d_count, void* stream);
-B200GS_API int b200gs_unpack_rows_grad(int64_t n, const int32_t* radii, const int32_t* offsets, const float* v_rows, float* v_xy,
-                                       float* v_depth, float* v_conic, float* v_comp, float* v_opacity, float* v_rgb, void* stream);
 /* block_counts / block_rows (optional; NULL / 0 = every row counts): the rows arrive in blocks of block_rows rows of which only the first
  *     block_counts[b] are valid (the fixed-capacity exchange of the sharded renderer) — the rest reads as culled, so the receive buffer
  *     needs no padding pass. */
